@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W            (N>1: launched under torchrun)
     python bench.py --impl reference --gpus N --steps K --warmup W
     python bench.py --gpus 1 --scale 27                      (the single-GPU denominator of the scale-27 configuration)
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR   (also writes the last timed step's result as .npy)
 
 Workload (BASELINE.json configs[1]): PageRank on RMAT scale-24 edge-factor-16 (Graph500 a,b,c,
 multi-edges and self-loops kept, scrambled ids, unweighted, int32 ids / float32 scores), alpha 0.85,
@@ -269,8 +270,7 @@ def run_single(args):
         return plc.pagerank(h, G, None, None, None, None, ALPHA, 0.0, ITERS, False, fail_on_nonconvergence=False)
 
     for _ in range(args.warmup):
-        v, p, _ = step()
-    nv = v.numel()
+        step()
     sampler = ClockSampler(0)
     torch.cuda.synchronize()
     sampler.start()
@@ -281,10 +281,14 @@ def run_single(args):
     e0.record(hstream)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        step()  # synchronous on return (the C-ABI syncs the handle's stream)
+        v, p, _ = step()  # synchronous on return (the C-ABI syncs the handle's stream)
     e1.record(hstream)
     torch.cuda.synchronize()
     wall = time.perf_counter() - t0
+    nv = v.numel()
+    if args.dump_outputs:
+        dump_pagerank(args.dump_outputs, v, p)
+    del v, p
     launches = h.launch_count() - l0
     clocks = sampler.stop()
     dev_s = e0.elapsed_time(e1) * 1e-3  # device time between the two events; wall is the host's view of the same region
@@ -405,6 +409,26 @@ def run_single(args):
     print(json.dumps(out), flush=True)
 
 
+DUMP_SAMPLE = 1 << 20
+
+
+def dump_pagerank(out_dir, verts, scores):
+    """The result of the last timed step, as its caller receives it (vertex ids, PageRank scores), sorted by vertex id so
+    that two builds that order their result rows differently compare row for row.  Above DUMP_SAMPLE vertices a fixed,
+    seeded sample of the sorted rows is written (8 + 4 bytes per row: at most 12 MB)."""
+    import numpy as np
+    import torch
+    order = torch.argsort(verts)
+    vs, ps = verts[order], scores[order]
+    if vs.numel() > DUMP_SAMPLE:
+        keep = np.sort(np.random.default_rng(0).choice(vs.numel(), DUMP_SAMPLE, replace=False))
+        idx = torch.as_tensor(keep, device=vs.device)
+        vs, ps = vs[idx], ps[idx]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "pagerank_vertices.npy"), vs.cpu().numpy().astype(np.float64))
+    np.save(os.path.join(out_dir, "pagerank_scores.npy"), ps.cpu().numpy().astype(np.float32))
+
+
 def _harmonic(xs):
     return len(xs) / sum(1.0 / x for x in xs) if xs else None
 
@@ -517,12 +541,18 @@ def main():
     ap.add_argument("--impl", default="b200")
     ap.add_argument("--scale", type=int, default=None, help="override RMAT scale (development only)")
     ap.add_argument("--cpu-sample-scale", type=int, default=22, help="RMAT scale of the cpu_baseline sample")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the vertices and scores of the last timed step to DIR/*.npy (single GPU)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl in ("reference", "cpu-sample"):
         pin_host_threads()  # before numpy / the oracle load an OpenMP runtime; ONLY in the CPU arms (see _cpu_baseline)
         return run_reference(args) if args.impl == "reference" else run_cpu_sample(args)
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if args.gpus > 1 or world > 1:
+        if args.dump_outputs:
+            ap.error("--dump-outputs is implemented for --gpus 1")
         return run_multi(args)  # weak scaling: scale 24 + log2(N); N = 8 is BASELINE's scale-27 configuration
     if args.scale is None:
         args.scale = 24

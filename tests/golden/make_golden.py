@@ -1,25 +1,30 @@
 #!/usr/bin/env python
-"""Generate tests/golden/*.json from the reference's own test fixtures (run in the build container,
-where /root/reference is mounted; the GPU box only ever reads the committed JSON).
+"""Generate tests/golden/reference_golden.json from the reference's own test fixtures (run where a checkout of
+the reference is available, named by $CUGRAPH_REFERENCE; the tests only ever read the committed JSON).
 
 Sources of truth (all read, none copied as source):
   * python/pylibcugraph/pylibcugraph/tests/test_pagerank.py  `_test_data`  (karate/dolphins/Simple_1/2)
   * python/pylibcugraph/pylibcugraph/tests/test_sssp.py      `_test_data`
-  * python/pylibcugraph/pylibcugraph/tests/conftest.py       Simple_1 / Simple_2 edge lists
-  * datasets/karate.csv, datasets/dolphins.csv               edge lists (data files)
+  * python/pylibcugraph/pylibcugraph/tests/conftest.py       Simple_1 / Simple_2 / invalid edge lists
+  * python/pylibcugraph/pylibcugraph/tests/test_{katz_centrality,eigenvector_centrality,connected_components}.py
+                                                             expected values (transcribed below with file:line)
+  * datasets/{karate,dolphins,toy_graph,toy_graph_undirected,karate-disjoint-sequential}.csv   edge lists
   * cpp/tests/c_api/{pagerank,bfs,sssp}_test.c               6-/4-vertex golden arrays (transcribed
     below with file:line, they are C array literals)
+  * cpp/tests/c_api/{pagerank,bfs,sssp,extract_paths,katz,hits,weakly_connected_components,eigenvector_centrality,
+    degrees}_test.c                                          every case's array literals and scalars (parsed)
 The pylibcugraph test modules import cupy; a numpy shim stands in for it here.
 """
 import importlib.util
 import json
 import os
+import re
 import sys
 import types
 
 import numpy as np
 
-REF = os.environ.get("CUGRAPH_REFERENCE", "/root/reference")
+REF = os.environ["CUGRAPH_REFERENCE"]
 OUT = os.path.dirname(os.path.abspath(__file__))
 
 
@@ -38,6 +43,55 @@ def _load_with_cupy_shim(path, name):
 def _csv(path):
     rows = [l.split() for l in open(path) if l.strip()]
     return ([int(r[0]) for r in rows], [int(r[1]) for r in rows], [float(r[2]) for r in rows])
+
+
+C_PROGRAMS = ["pagerank", "bfs", "sssp", "extract_paths", "katz", "hits", "weakly_connected_components",
+              "eigenvector_centrality", "degrees"]
+
+
+def _c_value(tok, arrays, scalars):
+    tok = tok.strip()
+    if tok in arrays:
+        return arrays[tok]
+    if tok in scalars:
+        return scalars[tok]
+    if tok in ("TRUE", "FALSE"):
+        return tok == "TRUE"
+    if tok == "NULL":
+        return None
+    if tok in ("FLT_MAX", "DBL_MAX"):
+        return tok
+    tok = tok.rstrip("fd") if re.fullmatch(r"[-+0-9.eE]+[fd]", tok) else tok
+    return float(tok) if re.search(r"[.eE]", tok) else int(tok)
+
+
+def _c_program_cases(path):
+    """The cases of one cpp/tests/c_api/*_test.c program, in the order its main() runs them: for each test function the
+    generic_* routine it returns into and that routine's arguments by parameter name (the host arrays and scalars the
+    test declares).  A test that does not delegate to a generic_* routine is recorded with the arrays and scalars it
+    declares."""
+    src = re.sub(r"/\*.*?\*/|//[^\n]*", "", open(path).read(), flags=re.S)
+    params = {}
+    for name, plist in re.findall(r"int\s+(generic_\w+)\s*\(([^)]*)\)\s*\{", src):
+        params[name] = [re.findall(r"\w+", p)[-1] for p in plist.split(",")]
+    bodies = dict(re.findall(r"int\s+(test_\w+)\s*\([^)]*\)\s*\{(.*?)\n\}", src, flags=re.S))
+    cases = []
+    for test in re.findall(r"RUN_TEST\((\w+)\)", src):
+        body = bodies[test]
+        arrays = {n: [_c_value(x, {}, {}) for x in v.replace("\n", " ").split(",") if x.strip()]
+                  for n, v in re.findall(r"\w+\s+(\w+)\[\]\s*=\s*\{([^}]*)\};", body)}
+        scalars = {n: _c_value(v, {}, {}) for n, v in
+                   re.findall(r"(?:size_t|double|float|bool_t|int|vertex_t|weight_t|edge_t)\s+(\w+)\s*=\s*([^;{]+);", body)}
+        call = re.search(r"return\s+(generic_\w+)\s*\((.*?)\);", body, flags=re.S)
+        case = {"name": test}
+        if call:
+            args = [_c_value(a, arrays, scalars) for a in call.group(2).split(",")]
+            case["generic"] = call.group(1)
+            case["args"] = dict(zip(params[call.group(1)], args))
+        else:
+            case["locals"] = dict(arrays, **scalars)
+        cases.append(case)
+    return cases
 
 
 def main():
@@ -65,6 +119,34 @@ def main():
                         "predecessors": np.asarray(ss._test_data[name]["predecessor"]).tolist(),
                         "predecessors_checked": name not in ("karate.csv", "dolphins.csv")}}
         out["pylibcugraph"][name] = ent
+
+    # test_katz_centrality.py:11,89-95 (datasets/toy_graph_undirected.csv) and test_eigenvector_centrality.py:16,85-90
+    # (datasets/toy_graph.csv)
+    ks, kd, kw = _csv(os.path.join(REF, "datasets/toy_graph_undirected.csv"))
+    es, ed, ew = _csv(os.path.join(REF, "datasets/toy_graph.csv"))
+    out["pylibcugraph_centralities"] = {
+        "katz": {"src": ks, "dst": kd, "weights": kw, "rel_tol": 1e-4,
+                 "alpha": 0.01, "beta": 1.0, "epsilon": 1e-6, "max_iterations": 1000,
+                 "values": [0.410614, 0.403211, 0.390689, 0.415175, 0.395125, 0.433226]},
+        "eigenvector": {"src": es, "dst": ed, "weights": ew, "rel_tol": 1e-4, "epsilon": 1e-6, "max_iterations": 200,
+                        "values": [0.236325, 0.292055, 0.458457, 0.60533, 0.190498, 0.495942]},
+    }
+    # test_connected_components.py:19-149: inputs (dense adjacency or an edge-list file) and the expected weak components
+    ks, kd, _ = _csv(os.path.join(REF, "datasets/karate-disjoint-sequential.csv"))
+    dolphins = graphs["dolphins.csv"]
+    out["pylibcugraph_wcc"] = {
+        "graph1": {"adjacency": [[0, 1, 1, 0, 0], [0, 0, 1, 0, 0], [0, 0, 0, 0, 0], [0, 0, 0, 0, 1], [0, 0, 0, 0, 0]],
+                   "components": [[0, 1, 2], [3, 4]]},
+        "graph2": {"adjacency": [[0, 1, 1, 0, 0], [1, 0, 1, 0, 0], [1, 1, 0, 0, 0], [0, 0, 0, 0, 1], [0, 0, 0, 1, 0]],
+                   "components": [[0, 1, 2], [3, 4]]},
+        "karate-disjoint-sequential": {"src": ks, "dst": kd, "components": [list(range(34)), [34, 35, 36]]},
+        "dolphins": {"src": dolphins[0], "dst": dolphins[1], "components": [list(range(62))]},
+    }
+    # conftest.py:25-37: edge lists SGGraph must reject with ValueError
+    out["pylibcugraph_invalid_graphs"] = {
+        "InvalidNumWeights_1": {"src": [0, 1, 2], "dst": [1, 2, 3], "weights": [1.0, 1.0, 1.0, 1.0]},
+        "InvalidNumVerts_1": {"src": [1, 2], "dst": [1, 2, 3], "weights": [1.0, 1.0, 1.0]},
+    }
 
     g6 = {"src": [0, 1, 1, 2, 2, 2, 3, 4], "dst": [1, 3, 4, 0, 1, 3, 5, 5],
           "weights": [0.1, 2.1, 1.1, 5.1, 3.1, 4.1, 7.2, 3.2], "num_vertices": 6}
@@ -98,6 +180,9 @@ def main():
         "sssp_6": dict(g6, source=0, cutoff=10.0,
                        distances=[0.0, 0.1, "MAX", 2.2, 1.2, 4.4], predecessors=[-1, 0, -1, 1, 1, 4]),
     }
+    # cpp/tests/c_api/<program>_test.c: every case of the C-API test programs, with the arguments of the generic_* routine
+    # it runs (inputs, parameters and expected results)
+    out["c_api_programs"] = {p: _c_program_cases(os.path.join(REF, "cpp/tests/c_api", f"{p}_test.c")) for p in C_PROGRAMS}
     with open(os.path.join(OUT, "reference_golden.json"), "w") as f:
         json.dump(out, f, indent=1)
     print("wrote", os.path.join(OUT, "reference_golden.json"))

@@ -71,14 +71,16 @@ def test_wrappers_match_oracle(surface):
     assert np.array_equal(gs, rs)
 
 
-def test_bench_single_gpu_arm(surface, monkeypatch, capsys):
-    """bench.run_single end to end at a toy scale: one JSON line with every key of the contract, including the BFS / SSSP
-    numbers as flat keys of `config` (the driver keeps `config`) and the CPU port + NetworkX baselines."""
+def test_bench_single_gpu_arm(surface, monkeypatch, capsys, tmp_path):
+    """bench.run_single end to end at a toy scale: one JSON line with every key of the result, including the BFS / SSSP
+    numbers as flat keys of `config` and the CPU port + NetworkX baselines; --dump-outputs writes the last timed step's
+    PageRank result."""
     monkeypatch.setenv("CUGRAPH_B200_SWEEP_MIN_EDGES", "0")
     monkeypatch.setenv("CUGRAPH_B200_BENCH_BFS_SOURCES", "3")
     monkeypatch.setenv("CUGRAPH_B200_BENCH_SSSP_SOURCES", "2")
     bench = _load(os.path.join(ROOT, "bench.py"), "bench_under_test")
-    args = argparse.Namespace(gpus=1, steps=2, warmup=1, impl="b200", scale=10, cpu_sample_scale=10)
+    args = argparse.Namespace(gpus=1, steps=2, warmup=1, impl="b200", scale=10, cpu_sample_scale=10,
+                              dump_outputs=str(tmp_path / "dump"))
     bench.run_single(args)
     line = [ln for ln in capsys.readouterr().out.splitlines() if ln.startswith("{")][-1]
     out = json.loads(line)
@@ -99,6 +101,11 @@ def test_bench_single_gpu_arm(surface, monkeypatch, capsys):
     assert cfg["bfs_sources"] == 3 and cfg["sssp_sources"] == 2
     for k in ("bfs_harmonic_mteps", "bfs_mean_mteps", "bfs_ms_per_source", "sssp_harmonic_mteps", "sssp_mean_mteps", "sssp_ms_per_source"):
         assert cfg[k] > 0, k
+    verts = np.load(tmp_path / "dump" / "pagerank_vertices.npy")
+    scores = np.load(tmp_path / "dump" / "pagerank_scores.npy")
+    assert verts.dtype == np.float64 and scores.dtype == np.float32
+    assert verts.size == scores.size == cfg["num_vertices"] and (np.diff(verts) > 0).all()
+    assert abs(float(scores.astype(np.float64).sum()) - 1.0) < 1e-4
 
 
 def test_bench_reference_arm(capsys):

@@ -1,16 +1,16 @@
-"""The reference's OWN C-API tests for this path — cpp/tests/c_api/{pagerank,bfs,sssp,extract_paths,katz,hits,weakly_connected_components,eigenvector_centrality,degrees}_test.c, compiled unmodified from
-where they lie under /root/reference against this repository's headers (oracle/ref_ctests/build.sh) — run here against the
-CPU emulation build of the library: every golden vector and error contract those programs check (pagerank_test.c:385-540,
-bfs_test.c:108-209, sssp_test.c:167-225) through the real C ABI.  Skipped where the reference sources are absent (the GPU
-box); tests/test_reference_c_tests_gpu.py runs the same programs linked against the CUDA library."""
+"""The reference's own C-API test programs for this path — cpp/tests/c_api/{pagerank,bfs,sssp,extract_paths,katz,hits,
+weakly_connected_components,eigenvector_centrality,degrees}_test.c — replayed case by case (tests/c_api_replay.py, from the
+cases recorded in tests/golden/reference_golden.json) against the CPU emulation build of the library: every golden vector
+and error contract those programs check, through the real C ABI.  tests/test_reference_c_tests_gpu.py replays the same
+cases against the CUDA library."""
 import os
-import subprocess
 import sys
 
 import pytest
 
+from tests.c_api_replay import run_program
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = os.environ.get("REF", "/root/reference")
 
 EXPECTED = {
     "pagerank": ["test_pagerank", "test_pagerank_with_transpose", "test_pagerank_4", "test_pagerank_4_with_transpose",
@@ -28,31 +28,24 @@ EXPECTED = {
 }
 
 
-def check_output(name, r):
-    assert r.returncode == 0, r.stdout + r.stderr
-    lines = [ln for ln in r.stdout.splitlines() if ln.startswith("RUNNING:")]
-    assert len(lines) == len(EXPECTED[name]), r.stdout
-    for case, ln in zip(EXPECTED[name], lines):
-        assert ln.startswith(f"RUNNING: {case}...") and ln.endswith("- passed"), ln
-    assert "ASSERTION FAILED" not in r.stdout
+def check_program(lib_path, golden, name):
+    """every case of the program passes, and the cases are the ones the program runs"""
+    results = run_program(lib_path, golden["c_api_programs"][name])
+    assert [case for case, _ in results] == EXPECTED[name]
+    failed = [f"{case}: {why}" for case, why in results if why is not None]
+    assert not failed, "\n".join(failed)
 
 
 @pytest.fixture(scope="module")
-def binaries():
-    if not os.path.isdir(os.path.join(REF, "cpp", "tests", "c_api")):
-        pytest.skip("reference sources not present")
+def emu_lib():
     sys.path.insert(0, os.path.join(ROOT, "emu"))
     import build_emu
     try:
-        lib = build_emu.build()
+        return build_emu.build()
     except Exception as e:
         pytest.skip(f"emulation build unavailable: {e}")
-    r = subprocess.run(["bash", os.path.join(ROOT, "oracle", "ref_ctests", "build.sh"), lib], capture_output=True, text=True)
-    assert r.returncode == 0, r.stdout + r.stderr
-    return os.path.join(ROOT, "oracle", "_ref")
 
 
 @pytest.mark.parametrize("name", ["pagerank", "bfs", "sssp", "extract_paths", "katz", "hits", "weakly_connected_components", "eigenvector_centrality", "degrees"])
-def test_reference_c_test_program(binaries, name):
-    r = subprocess.run([os.path.join(binaries, f"ref_{name}_test")], capture_output=True, text=True, timeout=300)
-    check_output(name, r)
+def test_reference_c_test_program(emu_lib, golden, name):
+    check_program(emu_lib, golden, name)

@@ -1,21 +1,14 @@
-"""The reference's own C-API test programs (cpp/tests/c_api/{pagerank,bfs,sssp,extract_paths,katz,hits,weakly_connected_components,eigenvector_centrality,degrees}_test.c, unmodified) linked against the CUDA
-library: built where the reference sources exist (__graft_entry__.build() -> oracle/ref_ctests/build.sh ... _gpu, outputs in
-oracle/_ref/, which travels to the GPU box) and run here on the B200.  (eigenvector_centrality_test.c and degrees_test.c:
-tests/test_zz_late_additions_gpu.py.)"""
-import os
-import subprocess
-
+"""The reference's own C-API test programs (cpp/tests/c_api/{pagerank,bfs,sssp,extract_paths,katz,hits,
+weakly_connected_components}_test.c) replayed case by case against the CUDA library on the B200 (tests/c_api_replay.py).
+(eigenvector_centrality_test.c and degrees_test.c: tests/test_zz_late_additions_gpu.py.)"""
 import pytest
 
-from tests.test_reference_c_tests_cpu import ROOT, check_output
+from cugraph_b200.build import LIB
+from tests.test_reference_c_tests_cpu import check_program
 
 pytestmark = pytest.mark.gpu
 
 
 @pytest.mark.parametrize("name", ["pagerank", "bfs", "sssp", "extract_paths", "katz", "hits", "weakly_connected_components"])
-def test_reference_c_test_program_on_gpu(name):
-    exe = os.path.join(ROOT, "oracle", "_ref", f"ref_{name}_test_gpu")
-    if not os.path.exists(exe):
-        pytest.skip("oracle/_ref/ref_*_test_gpu not built (needs the reference sources at build time)")
-    r = subprocess.run([exe], capture_output=True, text=True, timeout=300)
-    check_output(name, r)
+def test_reference_c_test_program_on_gpu(golden, name):
+    check_program(LIB, golden, name)

@@ -1,25 +1,18 @@
-"""GPU tests of the entry points that were added AFTER the round's last GPU call (validated under the emulation and by the
-reference's own test programs on CPU only): eigenvector centrality and the degree functions.  The file name sorts last on
-purpose: under `pytest -x` everything that has already run on hardware runs first."""
-import os
-import subprocess
-
+"""GPU tests of eigenvector centrality and the degree functions, the entry points added last.  The file name sorts last on
+purpose: under `pytest -x` the longer-standing GPU tests run first."""
 import numpy as np
 import pytest
 
-from tests.test_reference_c_tests_cpu import ROOT, check_output
+from cugraph_b200.build import LIB
+from tests.test_reference_c_tests_cpu import check_program
 from tests.test_siblings_gpu import _graph
 
 pytestmark = pytest.mark.gpu
 
 
 @pytest.mark.parametrize("name", ["eigenvector_centrality", "degrees"])
-def test_reference_c_test_program_on_gpu(name):
-    exe = os.path.join(ROOT, "oracle", "_ref", f"ref_{name}_test_gpu")
-    if not os.path.exists(exe):
-        pytest.skip("oracle/_ref/ref_*_test_gpu not built (needs the reference sources at build time)")
-    r = subprocess.run([exe], capture_output=True, text=True, timeout=300)
-    check_output(name, r)
+def test_reference_c_test_program_on_gpu(golden, name):
+    check_program(LIB, golden, name)
 
 
 def test_eigenvector_centrality_gpu():
