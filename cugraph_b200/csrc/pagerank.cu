@@ -4,7 +4,8 @@
 // Per iteration the reference runs ~6 V-sized thrust passes and 2 blocking scalar read-backs
 // (pagerank_impl.cuh:225-318).  Here an iteration is: pull sweep (spmv.cuh) -> [personalization
 // scatter] -> ONE fused vertex pass (diff, dangling sum, next x = pr/out_w) -> 1-thread finalize that
-// advances the device-resident loop state.  The host enqueues iterations in batches and only reads the
+// advances the device-resident loop state; on the piece stream without personalization everything after the sweep is one
+// kernel (k_pagerank_finish).  The host enqueues iterations in batches and only reads the
 // `done` flag between batches; kernels of iterations past convergence are no-ops, so the iteration
 // count and result are exactly those of a check-every-iteration loop.
 #include "sweep.cuh"
@@ -84,21 +85,125 @@ k_vertex_pass(T const* __restrict__ pr_new, T const* __restrict__ pr_old, T cons
   }
 }
 
-// advance the loop state (pagerank_impl.cuh:256-259, 320-329)
-__global__ void k_finalize(pr_state_t* st, double alpha, double epsilon, int n_vertices, int personalized,
-                           int count_iteration, int max_iterations)
+// advance the loop state (pagerank_impl.cuh:256-259, 320-329) from the iteration's diff and dangling sums
+__device__ __forceinline__ void advance_state(pr_state_t* st, double diff, double dangling, double alpha, double epsilon,
+                                              int n_vertices, int personalized, int count_iteration, int max_iterations)
 {
-  if (st->done) return;
-  double base    = st->dangling * alpha + (1.0 - alpha);
+  double base    = dangling * alpha + (1.0 - alpha);
   st->init       = personalized ? 0.0 : base / (double)n_vertices;
   st->pers_scale = base;
   if (count_iteration) {
     st->iter += 1;
-    st->last_diff = st->diff;
-    if (st->diff < epsilon || st->iter >= max_iterations) st->done = 1;
+    st->last_diff = diff;
+    if (diff < epsilon || st->iter >= max_iterations) st->done = 1;
   }
   st->diff     = 0.0;
   st->dangling = 0.0;
+}
+
+__global__ void k_finalize(pr_state_t* st, double alpha, double epsilon, int n_vertices, int personalized,
+                           int count_iteration, int max_iterations)
+{
+  if (st->done) return;
+  advance_state(st, st->diff, st->dangling, alpha, epsilon, n_vertices, personalized, count_iteration, max_iterations);
+}
+
+template <typename T> struct vec2_of;
+template <> struct vec2_of<float> { using type = float2; };
+template <> struct vec2_of<double> { using type = double2; };
+
+// The rest of a non-personalized PageRank iteration after k_sweep, in one pass over the rows (= vertices: the pull view has
+// no row_vertex): pr_new = acc * alpha + init, x = pr_new / out_w (pr_new where out_w == 0), diff += |pr_new - pr_old|,
+// dangling += pr_new where out_w == 0; clears the accumulators and the sweep's cursors.  The last CTA to finish (a ticket)
+// advances the loop state as k_finalize does.  This is k_sweep_finish + k_vertex_pass + k_finalize without the round trip of
+// pr_new through memory and without two launches per iteration.  Rows are read as in k_sweep_finish (a warp tile is
+// kPrSteps steps of 64 consecutive rows, lane = two rows, every load of a tile issued before the first use); the grid is a
+// few CTAs per SM, all resident, that stride over the tiles, so that only those few CTAs add their sums to the state and take a ticket.
+template <typename T>
+constexpr int pr_steps() { return 16 / (int)sizeof(T); }  // 4 (float) / 2 (double): the registers of 3 CTAs per SM
+constexpr int kPrCtasPerSm = 3;
+
+template <typename T>
+__global__ void __launch_bounds__(256, kPrCtasPerSm)  // all CTAs of the grid resident at once
+k_pagerank_finish(double* __restrict__ acc, int n_cov, int n_rows, T* __restrict__ pr_new, T const* __restrict__ pr_old,
+                  T const* __restrict__ out_w, T* __restrict__ x, int* __restrict__ cursor, int n_phases, double alpha,
+                  double epsilon, int max_iterations, pr_state_t* __restrict__ st)
+{
+  using T2 = typename vec2_of<T>::type;
+  constexpr int kPrSteps = pr_steps<T>();
+  __shared__ double s_red[2][8];
+  if (st->done) return;
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n_phases; i += gridDim.x * blockDim.x) cursor[i] = 0;
+  const int lane    = threadIdx.x & 31;
+  const int n_warps = gridDim.x * (blockDim.x >> 5);
+  const int n_tiles = (n_rows + 64 * kPrSteps - 1) / (64 * kPrSteps);
+  const double init = st->init;
+  double diff = 0.0, dang = 0.0;
+  for (int tile = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); tile < n_tiles; tile += n_warps) {
+    const int base = tile * (64 * kPrSteps) + 2 * lane;  // first of this lane's two rows in step 0
+    double2 q[kPrSteps];
+    T2 old[kPrSteps], ow[kPrSteps];
+#pragma unroll
+    for (int k = 0; k < kPrSteps; ++k) {
+      const int r = base + 64 * k;
+      q[k]        = make_double2(0.0, 0.0);
+      if (r + 1 < n_cov) q[k] = *reinterpret_cast<double2 const*>(acc + r);
+      else if (r < n_cov) q[k].x = acc[r];
+      old[k] = T2{(T)0, (T)0};
+      ow[k]  = T2{(T)0, (T)0};
+      if (r + 1 < n_rows) {
+        old[k] = *reinterpret_cast<T2 const*>(pr_old + r);
+        ow[k]  = *reinterpret_cast<T2 const*>(out_w + r);
+      } else if (r < n_rows) {
+        old[k].x = pr_old[r];
+        ow[k].x  = out_w[r];
+      }
+    }
+#pragma unroll
+    for (int k = 0; k < kPrSteps; ++k) {
+      const int r = base + 64 * k;
+      if (r + 1 < n_cov) *reinterpret_cast<double2*>(acc + r) = make_double2(0.0, 0.0);
+      else if (r < n_cov) acc[r] = 0.0;
+      if (r >= n_rows) continue;
+      const T v0 = (T)(q[k].x * alpha + init), v1 = (T)(q[k].y * alpha + init);
+      const T x0 = (ow[k].x == (T)0) ? v0 : v0 / ow[k].x, x1 = (ow[k].y == (T)0) ? v1 : v1 / ow[k].y;
+      diff += fabs((double)v0 - (double)old[k].x);
+      if (ow[k].x == (T)0) dang += (double)v0;
+      if (r + 1 < n_rows) {
+        diff += fabs((double)v1 - (double)old[k].y);
+        if (ow[k].y == (T)0) dang += (double)v1;
+        *reinterpret_cast<T2*>(pr_new + r) = T2{v0, v1};
+        *reinterpret_cast<T2*>(x + r)      = T2{x0, x1};
+      } else {
+        pr_new[r] = v0;
+        x[r]      = x0;
+      }
+    }
+  }
+  diff = warp_sum(diff);
+  dang = warp_sum(dang);
+  if (lane == 0) {
+    s_red[0][threadIdx.x >> 5] = diff;
+    s_red[1][threadIdx.x >> 5] = dang;
+  }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    double d = 0.0, g = 0.0;
+    for (int w = 0; w < (int)(blockDim.x >> 5); ++w) {
+      d += s_red[0][w];
+      g += s_red[1][w];
+    }
+    atomicAdd(&st->diff, d);
+    atomicAdd(&st->dangling, g);
+    __threadfence();  // the sums are visible before the ticket that counts them
+    if (atomicAdd(&st->ticket, 1u) == gridDim.x - 1) {
+      __threadfence();
+      volatile pr_state_t const* vs = st;  // every CTA's sums, not a cached copy
+      const double sum_diff = vs->diff, sum_dang = vs->dangling;
+      advance_state(st, sum_diff, sum_dang, alpha, epsilon, n_rows, 0, 1, max_iterations);
+      st->ticket = 0;
+    }
+  }
 }
 
 template <typename T>
@@ -287,16 +392,28 @@ void pagerank_typed(handle_impl const& h, graph_impl& g, pr_args const& a, centr
   if (max_it == 0) {
     // the reference's loop body runs at least once (pagerank_impl.cuh:224-327: test after iter++)
   }
+  // Non-personalized PageRank on the piece stream, rows = vertices (a graph stored transposed): k_sweep + k_pagerank_finish.
+  // Personalization scatters into pr_new between the sweep and the vertex pass, and with row_vertex the vertex-order streams
+  // would be gathered through it; those take the general path.
+  sweep_layout_t const* L = (!c.offs64 && n_pers == 0 && c.row_vertex.data() == nullptr && c.n_rows == nv)
+                              ? sweep_layout(h, c, nv, sizeof(T)) : nullptr;
+  const int fin_grid = std::max(std::min(ceil_div(nv, 64 * pr_steps<T>() * 8), h.sm_count * kPrCtasPerSm), 1);
   while (true) {
     int todo = std::min(batch, std::max(max_it, 1) - enqueued);
     for (int k = 0; k < todo; ++k) {
-      if (c.offs64) launch_pull_sweep<int64_t, T>(h, c, x.as<T>(), nxt, acc_hi.as<double>(), a.alpha, st);
-      else launch_pull_sweep_auto<int32_t, T>(h, c, nv, x.as<T>(), nxt, acc_hi.as<double>(), a.alpha, st);
-      if (n_pers > 0)
-        B200_LAUNCH(h, (k_personalize<T>), grid_for(n_pers), kBlock, 0, pers_idx.as<int32_t>(), (T const*)a.pers_val->data,
-                    n_pers, pers_sum, nxt, st);
-      B200_LAUNCH(h, (k_vertex_pass<T>), vgrid, kBlock, 0, nxt, cur, out_w, x.as<T>(), nv, st);
-      B200_LAUNCH(h, k_finalize, 1, 1, 0, st, a.alpha, a.epsilon, nv, n_pers > 0 ? 1 : 0, 1, max_it);
+      if (L) {
+        launch_sweep_pieces<T>(h, *L, x.as<T>(), acc_hi.as<double>(), st);
+        B200_LAUNCH(h, (k_pagerank_finish<T>), fin_grid, 256, 0, acc_hi.as<double>(), L->n_cov, nv, nxt,
+                    (T const*)cur, out_w, x.as<T>(), L->cursor.as<int>(), L->n_phases, a.alpha, a.epsilon, max_it, st);
+      } else {
+        if (c.offs64) launch_pull_sweep<int64_t, T>(h, c, x.as<T>(), nxt, acc_hi.as<double>(), a.alpha, st);
+        else launch_pull_sweep_auto<int32_t, T>(h, c, nv, x.as<T>(), nxt, acc_hi.as<double>(), a.alpha, st);
+        if (n_pers > 0)
+          B200_LAUNCH(h, (k_personalize<T>), grid_for(n_pers), kBlock, 0, pers_idx.as<int32_t>(), (T const*)a.pers_val->data,
+                      n_pers, pers_sum, nxt, st);
+        B200_LAUNCH(h, (k_vertex_pass<T>), vgrid, kBlock, 0, nxt, cur, out_w, x.as<T>(), nv, st);
+        B200_LAUNCH(h, k_finalize, 1, 1, 0, st, a.alpha, a.epsilon, nv, n_pers > 0 ? 1 : 0, 1, max_it);
+      }
       std::swap(cur, nxt);
       ++enqueued;
     }

@@ -31,6 +31,7 @@ struct pr_state_t {
   double last_diff;
   int iter;
   int done;
+  unsigned ticket;  // CTAs of k_pagerank_finish that are done with this iteration (the last one resets it)
 };
 
 #ifndef B200_HOST_EMU

@@ -633,10 +633,11 @@ k_sweep_finish(double* __restrict__ acc, int n_cov, int n_rows, T* __restrict__ 
   }
 }
 
+// k_sweep alone: acc[row] += the row's sum; the caller turns acc into its result and clears acc and the cursors.
 // x must hold padded_x_elems() elements, zero behind n_vertices (slices are copied whole)
 template <typename T>
-void launch_sweep(handle_impl const& h, csx_t const& c, sweep_layout_t const& L, T const* x, T* y, double* acc, double alpha,
-                  pr_state_t const* st, bool use_weights = true, bool covered_rows_only = false)
+void launch_sweep_pieces(handle_impl const& h, sweep_layout_t const& L, T const* x, double* acc, pr_state_t const* st,
+                         bool use_weights = true)
 {
   // the attribute is per device and cheap to set: no process-wide "done" flag (a second device would miss it)
   const bool weighted = use_weights && L.w.data() != nullptr;
@@ -659,6 +660,14 @@ void launch_sweep(handle_impl const& h, csx_t const& c, sweep_layout_t const& L,
   a.p.acc_pol = 0;
   if (weighted) B200_LAUNCH(h, (k_sweep<T, true>), L.n_cta, kSweepThreads, kSweepDynSmem, a);
   else B200_LAUNCH(h, (k_sweep<T, false>), L.n_cta, kSweepThreads, kSweepDynSmem, a);
+}
+
+// x must hold padded_x_elems() elements, zero behind n_vertices (slices are copied whole)
+template <typename T>
+void launch_sweep(handle_impl const& h, csx_t const& c, sweep_layout_t const& L, T const* x, T* y, double* acc, double alpha,
+                  pr_state_t const* st, bool use_weights = true, bool covered_rows_only = false)
+{
+  launch_sweep_pieces<T>(h, L, x, acc, st, use_weights);
   // 8 steps of 64 rows per warp: 0.335 ms per sweep against 0.340 with 4 and 0.354 with 2 (profiles/r02_fullchunk_ab.log)
   constexpr int kFinishSteps = 8;
   // covered_rows_only: y of the rows without edges already holds their (unvarying) value — multi-GPU blocks, where more than

@@ -337,6 +337,7 @@ template <typename T> inline T __reduce_add_sync(unsigned m, T v)
 }
 inline unsigned __activemask() { return 1u << emu_lane(); }  // worst-case divergence: every lane on its own
 inline void __syncwarp(unsigned m = 0xffffffffu) { unsigned long long out[32]; emu::warp_collect(m, 0ull, out); }
+inline void __threadfence() {}  // CTAs run one after the other: every write is visible
 inline void __syncthreads()
 {
   emu::cta_state_t& C = emu::cta();
